@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the legacy per-image scoring pass (BASELINE.json metric: images/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of B synthetic 24 MP frames per GPU:
 technical metrics (csrc/tech_stats.cu) + perceptual hash (csrc/phash.cu) + CLIP preprocess
@@ -53,7 +53,55 @@ def parse_args():
     ap.add_argument("--jpeg-restart-blocks", type=int, default=8, help="restart interval (MCUs) of the bench's JPEG streams")
     ap.add_argument("--e2e-jpeg-chunk", type=int, default=32, help="streams per decode launch in the JPEG e2e leg")
     ap.add_argument("--e2e-vit-batch", type=int, default=64, help="frames per ViT launch of the streamed e2e path")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step and the grouping stage computed (rank 0) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "facet_b200":
+        ap.error("--dump-outputs records the device path (--impl facet_b200)")
+    return args
+
+
+DUMP_BYTES = 64 * 1000 * 1000      # all files of --dump-outputs together
+
+
+def host_outputs(out, pairs, sims, hpairs):
+    """The device results of one step and of the grouping stage as float32 / float64 host arrays.  Integers become
+    float64 (exact: the technical sums of a 24 MP frame stay below 2^53); the 64-bit pHash becomes one 0/1 column per
+    bit, lowest first.  Pairs index the rows of all timed steps (step k, frame b -> k * batch + b) and are sorted."""
+    import numpy as np
+    arrays = {}
+    for name, t in out.items():
+        if t is None:
+            continue
+        a = t.cpu().numpy()
+        if name == "phash":
+            name, a = "phash_bits", (a.view(np.uint64)[:, None] >> np.arange(64, dtype=np.uint64)) & 1
+        arrays[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    cp = np.column_stack([pairs.cpu().numpy().astype(np.float64), sims.cpu().numpy().astype(np.float64)])
+    arrays["cosine_pairs"] = cp[np.lexsort((cp[:, 1], cp[:, 0]))]                 # rows (i, j, cosine)
+    hp = hpairs.cpu().numpy().astype(np.float64)
+    arrays["hamming_pairs"] = hp[np.lexsort((hp[:, 1], hp[:, 0]))]               # rows (i, j)
+    return arrays
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes out_dir/<name>.npy for every array, DUMP_BYTES in all: the smaller arrays are written whole first, and an
+    array that does not fit what is left keeps a seeded sample of its rows, in their order."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES
+    names = sorted(arrays, key=lambda k: arrays[k].nbytes)
+    for i, name in enumerate(names):
+        a = arrays[name]
+        share = left // (len(names) - i) - 4096          # room for the .npy header
+        if a.nbytes > share:
+            keep = np.random.default_rng(0).choice(len(a), share // (a.nbytes // len(a)), replace=False)
+            a = a[np.sort(keep)]
+        path = os.path.join(out_dir, name + ".npy")
+        np.save(path, a)
+        left -= os.path.getsize(path)
 
 
 def measured_peaks():
@@ -369,10 +417,10 @@ def main():
     def grouping(emb, hashes):
         """The duplicate-grouping stage over everything scored (configs[4]): ONE all-gather of the embedding shards and of
         the hashes, then every rank scans its balanced share of the pair triangle."""
-        pairs, _ = cosine_pairs_sharded(emb, 0.90)                 # bf16 gather -> scan, f32 gather overlapped -> recheck
+        pairs, sims = cosine_pairs_sharded(emb, 0.90)              # bf16 gather -> scan, f32 gather overlapped -> recheck
         h = all_gather_embeddings(hashes.view(-1, 1)).view(-1) if world > 1 else hashes
         hp = ops.hamming_pairs(h, 6, part=rank, nparts=world)      # duplicate rule of utils/duplicate.py:94-119
-        return pairs, hp
+        return pairs, sims, hp
 
     def barrier():
         if world > 1:
@@ -395,9 +443,9 @@ def main():
     sampler.reset()
     e0.record()
     for k in range(K):
-        step(k)
+        last = step(k)
     eg.record()
-    pairs, hpairs = grouping(emb_all, hash_all)
+    pairs, sims, hpairs = grouping(emb_all, hash_all)
     e1.record()
     barrier()
     ms_total = e0.elapsed_time(e1)
@@ -410,6 +458,8 @@ def main():
         ms_total, ms_group = (float(v) for v in t.tolist())
     ms_step = ms_total / K
     value = world * B * K / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, host_outputs(last, pairs, sims, hpairs))
 
     # ---- per-kernel device times of the SAME work: the library records a CUDA-event pair around each of its
     # launches on the launching stream (fb_profile_*); K more steps + grouping, identical inputs ----------------
@@ -562,7 +612,7 @@ def main():
         assert all("error" not in r for r in res_all), "e2e: a frame failed"
         emb = torch.from_numpy(np.frombuffer(b"".join(r["clip_embedding"] for r in res_all), dtype=np.float32).reshape(-1, 768).copy()).to(device)
         hh = torch.from_numpy(np.array([int(r["phash"], 16) for r in res_all], dtype=np.uint64).view(np.int64)).to(device)
-        p_, q_ = grouping(emb, hh)
+        p_, _, q_ = grouping(emb, hh)
         extra_h2d = emb.numel() * 4 + hh.numel() * 8
         extra_d2h = int(p_.cpu().numel() + q_.cpu().numel()) * 4
         barrier()
