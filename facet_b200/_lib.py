@@ -73,7 +73,6 @@ _SIGNATURES.update({
     "fb_f32_to_bf16": (C.c_int, [_P, _P, C.c_int64, _P]),
     "fb_cosine_pairs": (C.c_int, [_P, _P, C.c_int64, C.c_int, C.c_float, C.c_float, C.c_int64, C.c_int64, _P, _P,
                                   C.c_int64, _P, _P, _P, C.c_int64, _P, _P]),
-    "fb_cosine_candidates": (C.c_int, [_P, C.c_int64, C.c_int, C.c_float, C.c_int64, C.c_int64, _P, _P, C.c_int64, _P, _P]),
     "fb_cosine_block": (C.c_int, [_P, C.c_int64, C.c_int64, _P, C.c_int64, C.c_int64, C.c_int, C.c_float, C.c_int, _P, _P, C.c_int64, _P, _P]),
     "fb_cosine_recheck": (C.c_int, [_P, C.c_int, _P, _P, C.c_int64, C.c_float, _P, _P, C.c_int64, _P, _P]),
     "fb_vit_workspace_bytes": (C.c_size_t, [C.c_int]),

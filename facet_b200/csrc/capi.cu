@@ -370,19 +370,6 @@ int fb_cosine_pairs(const float* d_emb_f32, const void* d_emb_bf16, int64_t n, i
     return rc;
 }
 
-int fb_cosine_candidates(const void* d_emb_bf16, int64_t n, int dim, float threshold, int64_t row_offset, int64_t rows,
-                         int32_t* d_cand, float* d_cand_sims, int64_t cand_cap, uint64_t* d_cand_count, void* stream) {
-    FB_REQUIRE(n >= 1 && n < (1ll << 31) && d_cand_count, "fb_cosine_candidates: bad arguments");
-    cudaStream_t st = (cudaStream_t)stream;
-    FB_CUDA_OK(cudaMemsetAsync(d_cand_count, 0, sizeof(uint64_t), st));
-    if (rows <= 0 || n < 2) return 0;
-    ProfScope ps(PROF_COSINE, st);
-    int rc = launch_cosine_candidates(d_emb_bf16, dim, (int)n, (int)row_offset, (int)rows, dim, threshold, d_cand, d_cand_sims,
-                                      (long long)cand_cap, reinterpret_cast<unsigned long long*>(d_cand_count), st);
-    if (rc == 0) count_launch(1);
-    return rc;
-}
-
 int fb_cosine_block(const void* d_a_bf16, int64_t a_rows, int64_t a_offset, const void* d_b_bf16, int64_t b_rows, int64_t b_offset, int dim,
                     float threshold, int triangle, int32_t* d_cand, float* d_cand_sims, int64_t cand_cap, uint64_t* d_cand_count,
                     void* stream) {

@@ -21,8 +21,6 @@
 #include <mutex>
 #include <tuple>
 
-#include <cstdlib>
-
 #include "common.cuh"
 #include "kernels.h"
 #include "tc_common.cuh"
@@ -648,9 +646,8 @@ static int launch_cluster2(K kernel, int pairs, int threads, int smem_bytes, con
 }
 
 static int launch_gemm_common(const void* d_a, long long lda, const void* d_b, long long ldb, GemmArgs p, cudaStream_t stream) {
-    static const bool no_cluster = getenv("FB_GEMM_NO_CLUSTER") != nullptr;     // A/B switch
     // clusters of two with a multicast B tile: the ViT-layer GEMMs (large M, B = weights)
-    const bool cl2 = !no_cluster && p.mode != FB_GEMM_THRESHOLD_PAIRS && p.mode != FB_GEMM_F32 && p.M >= 4 * BM && p.N % BN == 0;
+    const bool cl2 = p.mode != FB_GEMM_THRESHOLD_PAIRS && p.mode != FB_GEMM_F32 && p.M >= 4 * BM && p.N % BN == 0;
     CUtensorMap ta, tb;
     int rc = make_tmap_bf16_2d(&ta, d_a, (uint64_t)p.M, (uint64_t)p.K, (uint64_t)lda, BM, BK);
     if (rc) return rc;

@@ -13,7 +13,6 @@
 // Host parsing of the marker segments and the table layout: facet_b200/utils/jpeg.py.
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "kernels.h"
@@ -454,8 +453,7 @@ __global__ void __launch_bounds__(kHuffThreads) jpeg_huffman_kernel(const uint8_
 //      more and stores coefficients, the DC ones as DIFFERENCES — also into a compact array, 2 bytes per block in scan order
 //      (jpeg_sync_write_kernel);
 //   5. a prefix sum per component over the compact array turns the differences into DC values (jpeg_dcx_segment_kernel), which
-//      the inverse DCT reads instead of coefficient 0 (FB_JPEG_DC_STRIDED: the same inside the coefficient area,
-//      jpeg_dc_segment_kernel).
+//      the inverse DCT reads instead of coefficient 0.
 #ifndef FB_SUBSEQ_BYTES
 #define FB_SUBSEQ_BYTES 512
 #endif
@@ -710,7 +708,7 @@ struct SyncArrays {
     const uint8_t* clean;
     long long clean_stride;
     int T;
-    int16_t* dc;             // [n][blocks per image] DC differences / values in scan order (compact DC integration), or nullptr
+    int16_t* dc;             // [n][blocks per image] DC differences / values in scan order (compact DC integration)
     long long dc_image_stride;
 };
 
@@ -876,7 +874,7 @@ __device__ bool span_write_coop(const uint8_t* u, long long len_bits, SyncState 
                         k = 0;
                         if (!skip) {
                             flush_blk = blk;
-                            if (dc_img) dc_img[q] = stage_row[0];        // compact copy of the DC difference, scan order
+                            dc_img[q] = stage_row[0];                    // compact copy of the DC difference, scan order
                         }
                         skip = false;
                         b = b + 1 == nblk ? 0 : b + 1;
@@ -938,68 +936,17 @@ __global__ void __launch_bounds__(kSyncWriteThreads) jpeg_sync_write_kernel(Sync
     const uint64_t lay = mcu_layout(g, nblk);
     const bool ok = span_write_coop(A.clean + (size_t)img * A.clean_stride, len_bits, st, limit, active, g, T, s_zz, lay, nblk, q, total_blocks,
                                     coef + (size_t)img * g.coef_image_stride, stage_warp, tid & 31,
-                                    A.dc ? A.dc + (size_t)img * A.dc_image_stride : nullptr);
+                                    A.dc + (size_t)img * A.dc_image_stride);
     if (!ok) atomicOr(status + img, 2);
 }
 
-// DC differences -> DC values: inclusive prefix sum over the blocks of one component in scan order, in segments of
-// kDcSeg blocks: (1) segment sums, (2) exclusive scan of the segment sums (one warp-sized loop per image and component),
-// (3) prefix inside each segment.  A thread owns 8 consecutive blocks, whose loads are issued together.
-constexpr int kDcPerThread = 8, kDcThreads = 256, kDcSeg = kDcPerThread * kDcThreads;
-
-__device__ __forceinline__ int16_t* dc_block_ptr(int16_t* base, const JpegGeom& g, int c, int j) {
-    const int per_mcu = g.hs[c] * g.vs[c];
-    const int m = j / per_mcu, r = j - m * per_mcu;
-    const int by = r / g.hs[c], bx = r - by * g.hs[c];
-    const int my = m / g.mcux, mx = m - my * g.mcux;
-    return base + ((size_t)(my * g.vs[c] + by) * g.blocks_w[c] + (mx * g.hs[c] + bx)) * 64;
-}
-
-// PHASE 0: seg_sum[img][c][seg] = sum of the segment's differences.  PHASE 1: the differences become values, starting from
-// seg_sum (then the exclusive prefix).  grid = (segments, n, ncomp)
-template <int PHASE>
-__global__ void __launch_bounds__(kDcThreads) jpeg_dc_segment_kernel(int16_t* __restrict__ coef, JpegGeom g, int segs, int* __restrict__ seg_sum) {
-    __shared__ int s_part[kDcThreads];
-    const int seg = blockIdx.x, img = blockIdx.y, c = blockIdx.z, tid = threadIdx.x;
-    int16_t* base = coef + (size_t)img * g.coef_image_stride + g.coef_comp_off[c];
-    const int count = g.mcux * g.mcuy * g.hs[c] * g.vs[c];
-    const int j0 = seg * kDcSeg + tid * kDcPerThread;
-    int16_t* ptr[kDcPerThread];
-    int v[kDcPerThread];
-#pragma unroll
-    for (int i = 0; i < kDcPerThread; ++i) {
-        ptr[i] = j0 + i < count ? dc_block_ptr(base, g, c, j0 + i) : nullptr;
-        v[i] = ptr[i] ? *ptr[i] : 0;
-    }
-    int sum = 0;
-#pragma unroll
-    for (int i = 0; i < kDcPerThread; ++i) sum += v[i];
-    s_part[tid] = sum;
-    __syncthreads();
-    for (int o = 1; o < kDcThreads; o <<= 1) {
-        const int x = tid >= o ? s_part[tid - o] : 0;
-        __syncthreads();
-        s_part[tid] += x;
-        __syncthreads();
-    }
-    int* ss = seg_sum + ((size_t)img * 3 + c) * segs;
-    if (PHASE == 0) {
-        if (tid == kDcThreads - 1) ss[seg] = s_part[tid];
-        return;
-    }
-    int run = ss[seg] + s_part[tid] - sum;
-#pragma unroll
-    for (int i = 0; i < kDcPerThread; ++i) {
-        run += v[i];
-        if (ptr[i]) *ptr[i] = (int16_t)run;
-    }
-}
-
-// Compact form of the same integration: the write pass also stores every block's DC difference at dc[img][q], q = index of the
-// block in scan order, so the prefix sums read and write 2 bytes per block contiguously instead of one 32-byte sector of the
-// coefficient area per block (twice), and the inverse DCT takes its DC term from this array.  A thread owns kDcxMcus
-// consecutive MCUs (nblk values each); segments of kDcxSeg MCUs; same three steps.  grid = (segments, n)
-constexpr int kDcxMcus = 8, kDcxSeg = kDcxMcus * kDcThreads;
+// DC differences -> DC values: inclusive prefix sum over the blocks of each component in scan order.  The write pass stores
+// every block's DC difference at dc[img][q], q = index of the block in scan order, so the prefix sums read and write 2 bytes per
+// block contiguously instead of one 32-byte sector of the coefficient area per block (twice), and the inverse DCT takes its DC
+// term from this array.  Segments of kDcxSeg MCUs: (1) segment sums (PHASE 0), (2) exclusive scan of the segment sums
+// (jpeg_dc_scan_kernel), (3) prefix inside each segment (PHASE 1).  A thread owns kDcxMcus consecutive MCUs (nblk values
+// each).  grid = (segments, n)
+constexpr int kDcThreads = 256, kDcxMcus = 8, kDcxSeg = kDcxMcus * kDcThreads;
 
 template <int PHASE>
 __global__ void __launch_bounds__(kDcThreads) jpeg_dcx_segment_kernel(int16_t* __restrict__ dc, long long dc_image_stride, JpegGeom g, int segs,
@@ -1292,15 +1239,15 @@ FB_HD void color_store8(const int (&yy)[8], const int (&cbv)[8], const int (&crv
     }
 }
 
-// MODE 0: chroma at full resolution (4:4:4); 1: h2v1 fancy; 2: h2v2 fancy.  Eight consecutive pixels x0 .. x0+7 (x0 a multiple
-// of 8) of row y of one image (P = its planes) -> 24 bytes at o.
+// MODE 0: chroma at full resolution (4:4:4); 1: h2v1 fancy (h2v2 frames take color_pair420).  Eight consecutive pixels
+// x0 .. x0+7 (x0 a multiple of 8) of row y of one image (P = its planes) -> 24 bytes at o.
 template <int MODE>
 FB_HD void color_group(const uint8_t* P, const JpegGeom& g, int y, int x0, int bgr, uint8_t* o) {
-    const int W = g.width, H = g.height;
+    static_assert(MODE == 0 || MODE == 1, "4:4:4 and h2v1 only: h2v2 frames are converted by color_pair420");
+    const int W = g.width;
     const int yp = g.blocks_w[0] * 8;                                   // plane pitches (multiples of 8)
     const int cp = g.ncomp == 3 ? g.blocks_w[1] * 8 : 0;
     const int cw = MODE == 0 ? W : (W + 1) / 2;                         // downsampled chroma size (ceil(size * samp / max))
-    const int ch = MODE == 2 ? (H + 1) / 2 : H;
     int yy[8], cbv[8], crv[8];
     {
         const uint2 w = *reinterpret_cast<const uint2*>(P + g.plane_comp_off[0] + (size_t)y * yp + x0);
@@ -1325,46 +1272,25 @@ FB_HD void color_group(const uint8_t* P, const JpegGeom& g, int y, int x0, int b
             }
         } else {
             const int c0 = x0 >> 1;
-            int sb[6], sr[6];                                   // per chroma column: the vertically filtered value
-            if (MODE == 1) {
-                chroma_cols(CB + (size_t)y * cp, c0, cw, sb);
-                chroma_cols(CR + (size_t)y * cp, c0, cw, sr);
-            } else {
-                const int cy = y >> 1;
-                int ny = (y & 1) ? cy + 1 : cy - 1;             // replicated context row at the top / bottom (jdmainct.c)
-                ny = ny < 0 ? 0 : (ny > ch - 1 ? ch - 1 : ny);
-                int a[6], b[6];
-                chroma_cols(CB + (size_t)cy * cp, c0, cw, a);
-                chroma_cols(CB + (size_t)ny * cp, c0, cw, b);
-#pragma unroll
-                for (int j = 0; j < 6; ++j) sb[j] = 3 * a[j] + b[j];
-                chroma_cols(CR + (size_t)cy * cp, c0, cw, a);
-                chroma_cols(CR + (size_t)ny * cp, c0, cw, b);
-#pragma unroll
-                for (int j = 0; j < 6; ++j) sr[j] = 3 * a[j] + b[j];
-            }
+            int sb[6], sr[6];
+            chroma_cols(CB + (size_t)y * cp, c0, cw, sb);
+            chroma_cols(CR + (size_t)y * cp, c0, cw, sr);
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
                 const int k = 1 + (j >> 1);                     // own chroma sample: column c0 + j / 2
                 const int nbk = (j & 1) ? k + 1 : k - 1;        // even pixel leans left, odd pixel leans right
-                if (MODE == 1) {
-                    const int bias = (j & 1) ? 2 : 1;
-                    cbv[j] = (3 * sb[k] + sb[nbk] + bias) >> 2;
-                    crv[j] = (3 * sr[k] + sr[nbk] + bias) >> 2;
-                } else {
-                    const int bias = (j & 1) ? 7 : 8;
-                    cbv[j] = (3 * sb[k] + sb[nbk] + bias) >> 4;
-                    crv[j] = (3 * sr[k] + sr[nbk] + bias) >> 4;
-                }
+                const int bias = (j & 1) ? 2 : 1;
+                cbv[j] = (3 * sb[k] + sb[nbk] + bias) >> 2;
+                crv[j] = (3 * sr[k] + sr[nbk] + bias) >> 2;
             }
         }
     }
     color_store8(yy, cbv, crv, g.ncomp == 3, bgr, W, x0, o);
 }
 
-// h2v2 frames, two rows per call: rows y (even) and y + 1 share their near chroma row y / 2 and differ only in the far row
-// (y / 2 - 1 above, y / 2 + 1 below, clamped), so a pair needs three chroma rows per plane instead of four and one set of
-// addresses.  Same arithmetic as color_group<2>.
+// h2v2 fancy upsampling, two rows per call: rows y (even) and y + 1 share their near chroma row y / 2 and differ only in the far
+// row (y / 2 - 1 above, y / 2 + 1 below, clamped: the replicated context row of jdmainct.c), so a pair needs three chroma rows
+// per plane instead of four and one set of addresses.
 FB_HD void color_pair420(const uint8_t* P, const JpegGeom& g, int y, int x0, int bgr, uint8_t* o) {
     const int W = g.width, H = g.height;
     const int yp = g.blocks_w[0] * 8, cp = g.blocks_w[1] * 8;
@@ -1511,8 +1437,7 @@ int launch_jpeg_decode(const uint8_t* d_bytes, const long long* d_scan_off, cons
     w += al((long long)chunks * 4 * n);
     const bool selfsync = g.restart_interval == 0 && total_mcus > kSerialMcus;
     const JpegTableSet* tables = reinterpret_cast<const JpegTableSet*>(d_tables);
-    const int16_t* dc_values = nullptr;          // set when the DC terms come from the compact array instead of coef[0]
-    long long dc_stride = 0;
+    const int16_t* dc_values = nullptr;          // DC values of the self-synchronising path; the restart-marker path leaves them in coef[0]
 
     FB_CUDA_OK(cudaMemsetAsync(d_status, 0, sizeof(int) * n, stream));
     if (selfsync) {
@@ -1537,8 +1462,7 @@ int launch_jpeg_decode(const uint8_t* d_bytes, const long long* d_scan_off, cons
         A.settled = reinterpret_cast<int*>(w);
         w += al(4ll * ((n + 63) & ~63));
         w += al(4ll * 3 * n * ((total_mcus * hmax * vmax + 2047) / 2048 + 1));          // segment sums of the DC integration
-        static const bool dc_strided = getenv("FB_JPEG_DC_STRIDED") != nullptr;          // A/B switch: integrate inside the coefficient area
-        A.dc = dc_strided ? nullptr : reinterpret_cast<int16_t*>(w);
+        A.dc = reinterpret_cast<int16_t*>(w);
         A.dc_image_stride = blocks;
         A.clean = clean;
         A.clean_len = clean_len;
@@ -1566,22 +1490,13 @@ int launch_jpeg_decode(const uint8_t* d_bytes, const long long* d_scan_off, cons
             jpeg_sync_write_kernel<<<dim3((A.T + kSyncWriteThreads - 1) / kSyncWriteThreads, n), kSyncWriteThreads, kSyncWriteSmem, stream>>>(
                 A, d_table_slot, tables, g, total_blocks, coef, d_status);
         }
-        if (A.dc) {
-            // compact DC integration: prefix sums over the 2-byte-per-block copy the write pass made; the inverse DCT reads it
-            const int segs = (int)((total_mcus + kDcxSeg - 1) / kDcxSeg);
-            int* seg_sum = reinterpret_cast<int*>(A.settled + ((n + 63) & ~63));
-            jpeg_dcx_segment_kernel<0><<<dim3(segs, n), kDcThreads, 0, stream>>>(A.dc, A.dc_image_stride, g, segs, seg_sum);
-            jpeg_dc_scan_kernel<<<n * 3, 32, 0, stream>>>(seg_sum, segs);
-            jpeg_dcx_segment_kernel<1><<<dim3(segs, n), kDcThreads, 0, stream>>>(A.dc, A.dc_image_stride, g, segs, seg_sum);
-            dc_values = A.dc;
-            dc_stride = A.dc_image_stride;
-        } else {
-            const int segs = (int)((g.mcux * (long long)g.mcuy * g.hs[0] * g.vs[0] + kDcSeg - 1) / kDcSeg);
-            int* seg_sum = reinterpret_cast<int*>(A.settled + ((n + 63) & ~63));
-            jpeg_dc_segment_kernel<0><<<dim3(segs, n, ncomp), kDcThreads, 0, stream>>>(coef, g, segs, seg_sum);
-            jpeg_dc_scan_kernel<<<n * 3, 32, 0, stream>>>(seg_sum, segs);
-            jpeg_dc_segment_kernel<1><<<dim3(segs, n, ncomp), kDcThreads, 0, stream>>>(coef, g, segs, seg_sum);
-        }
+        // compact DC integration: prefix sums over the 2-byte-per-block copy the write pass made; the inverse DCT reads it
+        const int segs = (int)((total_mcus + kDcxSeg - 1) / kDcxSeg);
+        int* seg_sum = reinterpret_cast<int*>(A.settled + ((n + 63) & ~63));
+        jpeg_dcx_segment_kernel<0><<<dim3(segs, n), kDcThreads, 0, stream>>>(A.dc, A.dc_image_stride, g, segs, seg_sum);
+        jpeg_dc_scan_kernel<<<n * 3, 32, 0, stream>>>(seg_sum, segs);
+        jpeg_dcx_segment_kernel<1><<<dim3(segs, n), kDcThreads, 0, stream>>>(A.dc, A.dc_image_stride, g, segs, seg_sum);
+        dc_values = A.dc;
     } else {
         if (g.n_intervals > 1) {
             dim3 grid(chunks, n);
@@ -1604,7 +1519,7 @@ int launch_jpeg_decode(const uint8_t* d_bytes, const long long* d_scan_off, cons
         long long gb = (total + 127) / 128;
         if (gb > (long long)sm_count() * 32) gb = (long long)sm_count() * 32;
         jpeg_idct_kernel<<<(unsigned)gb, 128, 0, stream>>>(coef, d_table_slot, reinterpret_cast<const JpegTableSet*>(d_tables), g, n, planes, dc_values,
-                                                           dc_stride);
+                                                           blocks);
     }
     {
         const int groups = (width + 7) / 8;
@@ -1613,11 +1528,7 @@ int launch_jpeg_decode(const uint8_t* d_bytes, const long long* d_scan_off, cons
         const int mode = ncomp == 1 ? 0 : (hmax == 1 ? 0 : (vmax == 1 ? 1 : 2));
         if (mode == 0) jpeg_color_kernel<0><<<grid, threads, 0, stream>>>(planes, g, n, bgr, d_out, out_stride);
         else if (mode == 1) jpeg_color_kernel<1><<<grid, threads, 0, stream>>>(planes, g, n, bgr, d_out, out_stride);
-        else {
-            static const bool single_rows = getenv("FB_JPEG_COLOR_SINGLE_ROWS") != nullptr;       // A/B switch
-            if (single_rows) jpeg_color_kernel<2><<<grid, threads, 0, stream>>>(planes, g, n, bgr, d_out, out_stride);
-            else jpeg_color420_pair_kernel<<<dim3((unsigned)((long long)n * ((height + 1) / 2)), grid.y), threads, 0, stream>>>(planes, g, n, bgr, d_out, out_stride);
-        }
+        else jpeg_color420_pair_kernel<<<dim3((unsigned)((long long)n * ((height + 1) / 2)), grid.y), threads, 0, stream>>>(planes, g, n, bgr, d_out, out_stride);
     }
     FB_CUDA_OK(cudaGetLastError());
     return 0;

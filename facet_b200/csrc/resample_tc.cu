@@ -19,8 +19,6 @@
 //             (about 64 B / clk / SM) is what bounds this pass.
 //   streaming (resample_h_tc_kernel) tile = (rows, block), coefficients loaded with every tile: shapes whose coefficient
 //             matrix does not fit beside the ring, or with more blocks than SMs.
-#include <cstdlib>
-
 #include "common.cuh"
 #include "kernels.h"
 #include "tc_common.cuh"
@@ -434,7 +432,6 @@ int launch_resample_h_tc(const uint8_t* d_images, int n, int H, int W, long long
     }
     // resident-coefficient schedule when the block's coefficient matrix fits beside a ring of >= 4 image stages
     {
-        static const bool no_resident = getenv("FB_RESAMPLE_STREAMING") != nullptr;      // A/B switch
         const int nblk = out_size / kNB;
         const int total_m = n * ((rows + RM - 1) / RM);
         const long long b_bytes = (long long)p.kblocks * RN * RKB;
@@ -443,7 +440,7 @@ int launch_resample_h_tc(const uint8_t* d_images, int n, int H, int W, long long
         if (stages > kResMaxStages) stages = kResMaxStages;
         int ngroups = sm_count() / nblk;
         if (ngroups > total_m) ngroups = total_m;
-        if (!no_resident && stages >= 4 && ngroups >= 1) {
+        if (stages >= 4 && ngroups >= 1) {
             ResidentArgs q;
             q.a = p;
             q.stages = stages;

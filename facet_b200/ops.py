@@ -422,37 +422,6 @@ def to_bf16(emb_f32):
     return out
 
 
-def cosine_pairs_split(emb_bf16, get_emb_f32, tau: float, part: int = 0, nparts: int = 1, band: float = 0.01, cap: int | None = None):
-    """cosine_pairs in two halves: the tensor-core scan runs on the bf16 matrix alone; `get_emb_f32()` is called only when the
-    float32 matrix is needed for the recheck (the multi-GPU flow passes a function that waits for an all-gather that was
-    running meanwhile).  Same results as cosine_pairs."""
-    torch = _lib.require_cuda()
-    lib = _lib.load()
-    eb = emb_bf16.contiguous()
-    n, d = eb.shape
-    bounds = balanced_row_blocks(n, nparts)
-    r0, r1 = bounds[part], bounds[part + 1]
-    e32 = None
-    with torch.cuda.device(eb.device):
-        cap = int(cap if cap is not None else max(1 << 20, 8 * n))      # 1 M candidates (12 MB): small, dense sets need no second pass
-        counts = torch.zeros(2, dtype=torch.int64, device=eb.device)
-        while True:
-            cand = torch.empty((cap, 2), dtype=torch.int32, device=eb.device)
-            cand_s = torch.empty((cap,), dtype=torch.float32, device=eb.device)
-            _lib.check(lib.fb_cosine_candidates(_ptr(eb), n, d, float(tau) - float(band), r0, r1 - r0, _ptr(cand), _ptr(cand_s), cap,
-                                                C.c_void_p(counts.data_ptr()), _lib.stream_ptr()), "fb_cosine_candidates")
-            if e32 is None:
-                e32 = get_emb_f32().contiguous()
-            pairs = torch.empty((cap, 2), dtype=torch.int32, device=eb.device)
-            sims = torch.empty((cap,), dtype=torch.float32, device=eb.device)
-            _lib.check(lib.fb_cosine_recheck(_ptr(e32), d, _ptr(cand), C.c_void_p(counts.data_ptr()), cap, float(tau), _ptr(pairs),
-                                             _ptr(sims), cap, C.c_void_p(counts.data_ptr() + 8), _lib.stream_ptr()), "fb_cosine_recheck")
-            nc, m = (int(x) for x in counts.tolist())
-            if nc <= cap and m <= cap:
-                return pairs[:m], sims[:m]
-            cap = _grown_cap(max(nc, m), 'cosine_pairs')
-
-
 def cosine_blocks(blocks, get_emb_f32, dim: int, tau: float, band: float = 0.01, cap: int | None = None, before_block=None):
     """Cosine pairs of a list of shard-against-shard blocks (the multi-GPU scan).  blocks: [(a_bf16 [m,dim], a_offset, b_bf16
     [n,dim], b_offset, triangle)] with GLOBAL row offsets; `before_block(k)` is called before block k is launched (the sharded

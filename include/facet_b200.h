@@ -288,18 +288,15 @@ int fb_cosine_pairs(const float* d_emb_f32, const void* d_emb_bf16, int64_t n, i
                     void* stream);
 
 /* The two halves of fb_cosine_pairs as separate calls, for the multi-GPU flow (utils/duplicate.py `cosine_pairs_sharded`):
- * the scan needs only the bf16 copy of the gathered matrix, so the all-gather of the float32 rows (twice the bytes) runs
- * on the NCCL stream WHILE the scan computes; the recheck waits for it.  fb_cosine_candidates emits (i, j, bf16 sim) with
- * sim >= threshold (= tau - band) for i in [row_offset, row_offset + rows), i < j; fb_cosine_recheck keeps the candidates
- * whose float64-accumulated dot product of the float32 rows is >= tau. */
-int fb_cosine_candidates(const void* d_emb_bf16, int64_t n, int dim, float threshold, int64_t row_offset, int64_t rows,
-                         int32_t* d_cand, float* d_cand_sims, int64_t cand_cap, uint64_t* d_cand_count, void* stream);
-/* One block of the all-pairs scan, for the multi-GPU flow in which every rank scans shard-against-shard blocks: the a_rows
- * rows at d_a_bf16 (global row index a_offset + i) against the b_rows rows at d_b_bf16 (global index b_offset + j), both
+ * the scan needs only bf16 rows, so the all-gather of the float32 rows (twice the bytes) runs on the NCCL stream WHILE the
+ * scan computes; the recheck waits for it.
+ * fb_cosine_block scans one shard-against-shard block and emits (i, j, bf16 sim) with sim >= threshold (= tau - band): the
+ * a_rows rows at d_a_bf16 (global row index a_offset + i) against the b_rows rows at d_b_bf16 (global index b_offset + j), both
  * [rows][dim] bf16 with row pitch dim.  triangle != 0 keeps only global column > global row (the block of a shard against
  * itself); rectangular blocks report every hit as (global row, global column) — the caller orders the pair.  Candidates are
  * APPENDED: d_cand_count is not reset, so a rank's blocks fill one list.  A rank can scan its own shard against itself while
- * the all-gather of the other shards is still in flight (utils/duplicate.py `cosine_pairs_sharded`). */
+ * the all-gather of the other shards is still in flight.
+ * fb_cosine_recheck keeps the candidates whose float64-accumulated dot product of the float32 rows is >= tau. */
 int fb_cosine_block(const void* d_a_bf16, int64_t a_rows, int64_t a_offset, const void* d_b_bf16, int64_t b_rows,
                     int64_t b_offset, int dim, float threshold, int triangle, int32_t* d_cand, float* d_cand_sims,
                     int64_t cand_cap, uint64_t* d_cand_count, void* stream);

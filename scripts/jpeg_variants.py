@@ -38,10 +38,7 @@ print(f"  {best:.2f} ms per 32 frames = {n / best * 1e3:.0f} frames/s, status {s
 '''
 for name in sys.argv[1:]:
     env = dict(os.environ)
-    if name.startswith("env:"):                       # env:VAR1,VAR2 -> the A/B switches of the library (read once per process)
-        for var in name[4:].split(","):
-            env[var] = "1"
-    elif name != "main":
+    if name != "main":
         env["FACET_B200_LIB"] = os.path.abspath(f"facet_b200/variants/lib_{name}.so")
     print(name, flush=True)
     subprocess.run([sys.executable, "-c", CHILD], env=env)

@@ -1,6 +1,5 @@
-"""CLIP preprocess and pHash on 24 MP frames (32 per launch, CUDA events, best of 3 x 3); FB_RESAMPLE_STREAMING=1 selects the
-streaming schedule of the tensor-core resampler for A/B runs."""
-import os, sys
+"""CLIP preprocess and pHash on 24 MP frames (32 per launch, CUDA events, best of 3 x 3)."""
+import sys
 import torch
 sys.path.insert(0, ".")
 sys.path.insert(0, "scripts")
@@ -29,4 +28,4 @@ def best_ms(fn):
 
 a = best_ms(lambda: ops.clip_preprocess(fr))
 b = best_ms(lambda: ops.phash(fr, device_only=True, luma=luma))
-print(f"{'streaming' if os.environ.get('FB_RESAMPLE_STREAMING') else 'resident '}: clip_preprocess {a * 1e3 / n:.2f} us / frame, phash (luma ready) {b * 1e3 / n:.2f} us / frame")
+print(f"clip_preprocess {a * 1e3 / n:.2f} us / frame, phash (luma ready) {b * 1e3 / n:.2f} us / frame")

@@ -182,25 +182,15 @@ int main(int argc, char** argv) {
             idct_block(coef + g.coef_comp_off[c] + b * 64, T_->q[g.tq[c]], planes + g.plane_comp_off[c] + (size_t)brow * 8 * bw * 8 + (size_t)bcol * 8,
                        (size_t)bw * 8);
         }
-    std::vector<uint8_t> out((size_t)g.width * g.height * 3 + 32);
+    std::vector<uint8_t> out((size_t)g.width * (g.height + 1) * 3 + 32);
     const int mode = g.ncomp == 1 ? 0 : (hmax == 1 ? 0 : (vmax == 1 ? 1 : 2));
-    for (int y = 0; y < g.height; ++y)
+    for (int y = 0; y < g.height; y += mode == 2 ? 2 : 1)
         for (int x0 = 0; x0 < g.width; x0 += 8) {
             uint8_t* o = out.data() + ((size_t)y * g.width + x0) * 3;
             if (mode == 0) color_group<0>(planes, g, y, x0, bgr, o);
             else if (mode == 1) color_group<1>(planes, g, y, x0, bgr, o);
-            else color_group<2>(planes, g, y, x0, bgr, o);
+            else color_pair420(planes, g, y, x0, bgr, o);
         }
-    if (mode == 2) {
-        // the row-pair form of the conversion (jpeg_color420_pair_kernel) must give the same frame
-        std::vector<uint8_t> out3((size_t)g.width * (g.height + 1) * 3 + 32);
-        for (int y = 0; y < g.height; y += 2)
-            for (int x0 = 0; x0 < g.width; x0 += 8) color_pair420(planes, g, y, x0, bgr, out3.data() + ((size_t)y * g.width + x0) * 3);
-        if (memcmp(out.data(), out3.data(), (size_t)g.width * g.height * 3) != 0) {
-            fprintf(stderr, "row-pair 4:2:0 conversion differs from the single-row result\n");
-            return 6;
-        }
-    }
     f = fopen(argv[2], "wb");
     fwrite(out.data(), 1, (size_t)g.width * g.height * 3, f);
     fclose(f);
