@@ -669,11 +669,14 @@ static int launch_gemm_common(const void* d_a, long long lda, const void* d_b, l
         else gemm_bf16_kernel<MODE_, false, false><<<grid, threads_, smem_, stream>>>(ta, tb, p);                      \
         break;                                                                                                         \
     }
+// Kernel attributes and the co-resident cluster count are per device (one process may drive several GPUs): a
+// PerDeviceFlag plus one pair count per device ordinal, the same pattern as sm_count().
 #define FB_LAUNCH_MODE_CL2(MODE_)                                                                                      \
     case MODE_: {                                                                                                      \
-        static int max_pairs = -1;                                                                                     \
+        static PerDeviceFlag attr_set;                                                                                 \
+        static std::atomic<int> max_pairs_dev[64];                                                                     \
         constexpr int threads_ = gemm_threads(MODE_, true), smem_ = gemm_smem_bytes(MODE_, true);                      \
-        if (max_pairs < 0) {                                                                                           \
+        if (!attr_set.get()) {                                                                                         \
             FB_CUDA_OK(cudaFuncSetAttribute(gemm_bf16_kernel<MODE_, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_)); \
             FB_CUDA_OK(cudaFuncSetAttribute(gemm_bf16_kernel<MODE_, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_)); \
             int a_ = 0, b_ = 0;                                                                                        \
@@ -681,8 +684,10 @@ static int launch_gemm_common(const void* d_a, long long lda, const void* d_b, l
             if (rc) return rc;                                                                                         \
             rc = max_cluster_pairs(gemm_bf16_kernel<MODE_, true, true>, threads_, smem_, &b_);                         \
             if (rc) return rc;                                                                                         \
-            max_pairs = a_ < b_ ? a_ : b_;                                                                             \
+            max_pairs_dev[PerDeviceFlag::device()].store(a_ < b_ ? a_ : b_, std::memory_order_relaxed);                \
+            attr_set.set();                                                                                            \
         }                                                                                                              \
+        const int max_pairs = max_pairs_dev[PerDeviceFlag::device()].load(std::memory_order_relaxed);                  \
         const int work_ = ((tiles_m + 1) / 2) * tiles_n;                                                               \
         const int pairs_ = work_ < max_pairs ? work_ : max_pairs;                                                      \
         FB_REQUIRE(pairs_ >= 1, "fb_gemm_bf16: no cluster of two CTAs fits on this device");                          \

@@ -22,8 +22,10 @@ import torch.nn.functional as F
 HEADS = 16
 
 
-def encode_image(sd: dict, x: torch.Tensor, layers: int | None = None) -> torch.Tensor:
-    """x [B,3,224,224] float32 -> un-normalised features [B,768] (open_clip encode_image)."""
+def encode_image(sd: dict, x: torch.Tensor, layers: int | None = None, return_tokens: bool = False):
+    """x [B,3,224,224] -> un-normalised features [B,768] (open_clip encode_image), in the dtype of x and sd
+    (float32, or float64 for an error yardstick).  return_tokens=True also returns the residual stream after
+    the last block, [B,257,1024]: (features, tokens)."""
     x = F.conv2d(x, sd["conv1.weight"], bias=None, stride=14)            # [B,1024,16,16]
     b, w = x.shape[0], x.shape[1]
     x = x.reshape(b, w, -1).permute(0, 2, 1)                              # [B,256,1024]
@@ -48,16 +50,20 @@ def encode_image(sd: dict, x: torch.Tensor, layers: int | None = None) -> torch.
         y = F.gelu(F.linear(y, sd[p + "mlp.c_fc.weight"], sd[p + "mlp.c_fc.bias"]))
         x = x + F.linear(y, sd[p + "mlp.c_proj.weight"], sd[p + "mlp.c_proj.bias"])
     pooled = F.layer_norm(x[:, 0], (w,), sd["ln_post.weight"], sd["ln_post.bias"], 1e-5)
-    return pooled @ sd["proj"]
+    return (pooled @ sd["proj"], x) if return_tokens else pooled @ sd["proj"]
 
 
-def score_batch(sd: dict, x: torch.Tensor, tag_embeddings: torch.Tensor | None = None):
-    """scorer.py:661-671: features -> (embedding, aesthetic in [0,10], raw, tag sims)."""
+def score_batch(sd: dict, x: torch.Tensor, tag_embeddings: torch.Tensor | None = None, return_tokens: bool = False):
+    """scorer.py:661-671: features -> (embedding, aesthetic in [0,10], raw, tag sims); return_tokens=True adds
+    "tokens", the residual stream after the last block [B,257,1024]."""
     with torch.no_grad():
-        feats = encode_image(sd, x)
+        feats, tokens = encode_image(sd, x, return_tokens=True)
         emb = F.normalize(feats, dim=-1)
-        h = F.relu(F.linear(feats.float(), sd["aesthetic_head.0.weight"], sd["aesthetic_head.0.bias"]))
+        h = F.relu(F.linear(feats, sd["aesthetic_head.0.weight"], sd["aesthetic_head.0.bias"]))
         raw = F.linear(h, sd["aesthetic_head.2.weight"], sd["aesthetic_head.2.bias"]).flatten()
         aesthetic = ((raw + 1) * 5).clamp(0.0, 10.0)
         sims = emb @ tag_embeddings.T if tag_embeddings is not None else None
-    return {"features": feats, "embedding": emb, "aesthetic": aesthetic, "aesthetic_raw": raw, "tag_sims": sims}
+    out = {"features": feats, "embedding": emb, "aesthetic": aesthetic, "aesthetic_raw": raw, "tag_sims": sims}
+    if return_tokens:
+        out["tokens"] = tokens
+    return out
