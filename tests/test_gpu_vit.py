@@ -1,7 +1,7 @@
 """GPU numerics for the tensor-core path: GEMM and attention against float64 truth computed from the exact 16-bit
-operands, at error bounds derived from the kernels' rounding steps; LayerNorm vs plain PyTorch fp32; the whole ViT-L/14
-tower + heads vs the fp32 oracle (north_star: cosine >= 0.999, aesthetic +-0.01).  tests/test_gpu_vit_f64.py checks
-the tower's whole residual stream against float64."""
+operands, at error bounds derived from the kernels' rounding steps; the whole ViT-L/14 tower + heads vs the fp32 oracle
+(north_star: cosine >= 0.999, aesthetic +-0.01).  tests/test_gpu_vit_f64.py checks the tower's whole residual stream
+against float64; tests/test_gpu_vit_heads_f64.py the tail, the stored-embedding heads, LayerNorm and im2col."""
 import numpy as np
 import pytest
 
@@ -174,22 +174,6 @@ def test_gemm_pair_kernel_on_two_devices():
         outs.append([t.cpu() for t in got + [out]])
     for x0, x1 in zip(*outs):
         assert torch.equal(x0, x1)
-
-
-def test_layernorm_and_assembly():
-    import torch
-    from facet_b200 import ops
-    x = torch.randn(1000, 1024, device="cuda") * 3 + 0.5
-    g, b = torch.randn(1024, device="cuda"), torch.randn(1024, device="cuda")
-    ref = torch.nn.functional.layer_norm(x, (1024,), g, b, 1e-5)
-    torch.testing.assert_close(ops.vit_layernorm(x, g, b, out_bf16=False), ref, rtol=1e-5, atol=1e-5)
-    torch.testing.assert_close(ops.vit_layernorm(x, g, b, out_bf16=True).float(), ref, rtol=1e-2, atol=1e-2)
-    pe = torch.randn(3 * 256, 1024, device="cuda")
-    cls, pos = torch.randn(1024, device="cuda"), torch.randn(257, 1024, device="cuda")
-    tok = torch.cat([cls.expand(3, 1, 1024), pe.reshape(3, 256, 1024)], 1) + pos
-    ref = torch.nn.functional.layer_norm(tok, (1024,), g, b, 1e-5).reshape(-1, 1024)
-    got = ops.vit_layernorm(pe, g, b, out_bf16=False, class_emb=cls, pos_emb=pos, rows=3 * 257)
-    torch.testing.assert_close(got, ref, rtol=1e-5, atol=1e-5)
 
 
 def _attn_truth(qkv, bsz):
@@ -375,19 +359,3 @@ def test_vit_tower_vs_fp32_oracle(dt, aest_tol):
     assert float((out["tag_sims"] - ref["tag_sims"]).abs().max()) <= 5e-3
     nrm = out["embedding"].norm(dim=-1)
     torch.testing.assert_close(nrm, torch.ones_like(nrm), rtol=1e-5, atol=1e-5)
-
-
-def test_embedding_heads_match_torch():
-    """fb_embedding_heads (score_from_embedding / tagger similarities on stored embeddings) vs plain fp32 PyTorch."""
-    import torch
-    from facet_b200 import ops
-    g = torch.Generator(device="cuda").manual_seed(4)
-    v = torch.nn.functional.normalize(torch.randn(5, 768, device="cuda", generator=g), dim=-1)
-    w1, b1 = torch.randn(256, 768, device="cuda", generator=g) * 768 ** -0.5, torch.randn(256, device="cuda", generator=g) * 0.02
-    w2, b2 = torch.randn(256, device="cuda", generator=g) * 256 ** -0.5, torch.randn(1, device="cuda", generator=g) * 0.02
-    tags = torch.nn.functional.normalize(torch.randn(240, 768, device="cuda", generator=g), dim=-1)
-    raw, sims = ops.embedding_heads(v, head=(w1, b1, w2, b2), tag_embeddings=tags)
-    ref_raw = torch.relu(v @ w1.T + b1) @ w2 + b2
-    torch.testing.assert_close(raw, ref_raw, rtol=1e-5, atol=1e-5)
-    torch.testing.assert_close(sims, v @ tags.T, rtol=1e-5, atol=1e-5)
-    assert ops.embedding_heads(v, tag_embeddings=tags)[0] is None and ops.embedding_heads(v, head=(w1, b1, w2, b2))[1] is None
